@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BAGEL-7B-MoT text->image denoising throughput on B200 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Workload (BASELINE.json configs[1], SURVEY.md §8d cfg 2): BAGEL-7B-MoT random-init, 1024x1024 (4096 latent tokens
@@ -59,7 +59,13 @@ def parse_args():
                          "gpu_library_baseline, parity, strong_scaling)")
     ap.add_argument("--blocks", default="attn,und,edit,library,strong",
                     help="comma list of extra blocks to run (default: all)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the latents they produced as DIR/<name>.npy (float32), so that "
+                         "two builds can be compared output for output on identical seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def measured_peaks():
@@ -253,6 +259,27 @@ def run_reference_arm(args):
 
 
 # ------------------------------------------------------------------------------------------------------
+DUMP_BYTES_MAX = 60 << 20       # all ranks together: stays under 64 MB with the .npy headers
+
+
+def dump_latents(out_dir: str, latents, rank: int, world: int):
+    """--dump-outputs: the per-sample latents x_t after the last timed step (what FlowRunner.latents() hands a
+    caller) as one float32 array [samples, tokens, 64]. Above this rank's share of DUMP_BYTES_MAX, a fixed seeded
+    subset of token rows [k, 64] in their original order, so every build stores the same elements."""
+    import numpy as np
+    import torch
+
+    x = torch.stack(latents, 0).float().cpu()
+    cap = DUMP_BYTES_MAX // world
+    if x.numel() * 4 > cap:
+        rows = x.reshape(-1, x.shape[-1])
+        k = cap // (rows.shape[1] * 4)
+        idx = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:k].sort().values
+        x = rows[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "latents.npy" if world == 1 else f"latents_rank{rank}.npy"), x.numpy())
+
+
 _JSON_FD = None
 
 
@@ -343,6 +370,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_per_step = float(t.item()) / args.steps
     value = (B * world) / (EVALS_PER_IMAGE * ms_per_step / 1000.0)
+    if args.dump_outputs:
+        dump_latents(args.dump_outputs, runner.latents(), rank, world)
     del runner
 
     # ---------------- roofline of the dominant kernel ----------------
